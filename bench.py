@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W            # this repo's CUDA path
     python bench.py --impl reference --gpus N --steps K --warmup W   # the CPU reference arm
+    python bench.py --gpus N --steps K --warmup W --dump-outputs DIR   # + the last timed step's top-k as .npy
 
 Workload (config.workload): BASELINE.json configs[1] -- 10M-doc synthetic MSMARCO-shaped corpus
 (searcharray_b200/synth.py, seeded, generated as postings), single-term BM25.  One "step" = one
@@ -465,6 +466,24 @@ def topk_of_dense(dense, k):
     return docs, scores
 
 
+DUMP_LIMIT_BYTES = 64 << 20
+
+
+def dump_outputs(out_dir, docs, scores):
+    """Writes the global top-k of the last timed step as <out_dir>/topk_docs.npy (float64 doc ids, exact;
+    0xFFFFFFFF = no doc) and topk_scores.npy (float32), one row per query, so that two builds can be compared
+    output for output.  Above 64 MB in all, a fixed seeded sample of the rows is written, with its row numbers
+    in topk_rows.npy."""
+    os.makedirs(out_dir, exist_ok=True)
+    rows = np.arange(docs.shape[0])
+    max_rows = (DUMP_LIMIT_BYTES - 4096) // (docs.shape[1] * (8 + 4) + 8)      # 4 KB for the .npy headers
+    if len(rows) > max_rows:
+        rows = np.sort(np.random.default_rng(0).choice(len(rows), max_rows, replace=False))
+        np.save(os.path.join(out_dir, "topk_rows.npy"), rows.astype(np.float64))
+    np.save(os.path.join(out_dir, "topk_docs.npy"), docs[rows].astype(np.float64))
+    np.save(os.path.join(out_dir, "topk_scores.npy"), scores[rows].astype(np.float32))
+
+
 def bench_ours(args, rank, world):
     from searcharray_b200 import synth
     o = Ours(args, rank, world)
@@ -497,6 +516,8 @@ def bench_ours(args, rank, world):
     dev_ms = o.timed_executes(args.steps)
     launches_value = int(o.stats().total_launches)
     o.download(out_docs, out_scores)
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, out_docs, out_scores)
     value = args.steps * Q / (dev_ms / 1e3)
     dbg("device-timed steps done")
 
@@ -626,7 +647,7 @@ def bench_ours(args, rank, world):
             o.upload(p_terms, p_starts, p_idf, slop, k); o.execute(); p_redo += o.download(p_docs, p_scores)
         dbg("  warm-up done, repairs", p_redo)
         o.upload(p_terms, p_starts, p_idf, slop, k)
-        p_steps = max(2, args.steps)
+        p_steps = args.steps
         p_ms = o.timed_executes(p_steps)
         dbg("  timed done")
         _lib.check(L.sa_stats_reset(h))
@@ -907,7 +928,11 @@ def main():
                          "(default 48 at 1 GPU, 16 sharded -- rank 0 then re-generates the FULL corpus; 0 = off)")
     ap.add_argument("--verify-phrases", type=int, default=12)
     ap.add_argument("--verify-edismax", type=int, default=2)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the top-k doc ids and scores of the last timed step as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of --impl ours")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     if args.impl == "reference":

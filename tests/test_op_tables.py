@@ -1,7 +1,7 @@
 """CPU: the oracle's C restatement of the reference's native ops (oracle/sa_oracle.c) against the
 known-answer tables of the reference's own op tests (test/test_snp_ops.py, test/test_bitcount64.py;
-extracted by tests/golden/make_golden_op_tables.py), and -- where the reference tree is present --
-against the reference's recorded output on its seven saved posting pairs."""
+extracted by tests/golden/make_golden_op_tables.py), and against the reference's output on samples of its
+seven saved posting pairs."""
 import hashlib
 import json
 import os
@@ -12,6 +12,7 @@ import pytest
 from conftest import GOLDEN
 
 T = json.load(open(os.path.join(GOLDEN, "op_tables.json")))
+P = np.load(os.path.join(GOLDEN, "posting_pairs.npz"))
 U = lambda xs: np.asarray(xs, dtype=np.uint64)
 
 
@@ -65,15 +66,17 @@ def test_bitcount_and_unique_tables():
 
 @pytest.mark.parametrize("sc", T["fixtures"], ids=[str(s["suffix"]) for s in T["fixtures"]])
 def test_saved_posting_pairs(sc):
-    """The reference's seven real posting pairs (fixtures/*.npy stay in the reference tree)."""
-    base = "/root/reference/fixtures"
-    if not os.path.exists(f"{base}/lhs_{sc['suffix']}.npy"):
-        pytest.skip("reference fixtures not present on this machine")
+    """The reference's seven real posting pairs, each kept whole up to 1,024 words a side and sampled to about
+    that size above it, with the reference's output on each (tests/golden/make_golden_posting_pairs.py)."""
     from oracle import ops
-    lhs, rhs = np.load(f"{base}/lhs_{sc['suffix']}.npy"), np.load(f"{base}/rhs_{sc['suffix']}.npy")
-    mask = np.uint64(sc["mask"])
-    assert (len(lhs), len(rhs)) == (sc["n_lhs"], sc["n_rhs"])
+    n = sc["suffix"]
+    lhs, rhs, mask = P[f"{n}.lhs"], P[f"{n}.rhs"], P[f"{n}.mask"][()]
+    assert mask == np.uint64(sc["mask"])
     li, ri = ops.intersect(lhs, rhs, mask=mask)
-    assert [len(li), digest(li), digest(ri)] == sc["intersect"]
+    assert np.array_equal(li, P[f"{n}.intersect.lhs_idx"]) and np.array_equal(ri, P[f"{n}.intersect.rhs_idx"])
     got = ops.intersect_with_adjacents(lhs, rhs, mask=mask)
-    assert [[len(x), digest(x)] for x in got] == sc["with_adjacents"]
+    for i, g in enumerate(got):
+        assert np.array_equal(g, P[f"{n}.with_adjacents.{i}"]), i
+    if (len(lhs), len(rhs)) == (sc["n_lhs"], sc["n_rhs"]):        # a whole pair: the digests of the full output too
+        assert [len(li), digest(li), digest(ri)] == sc["intersect"]
+        assert [[len(x), digest(x)] for x in got] == sc["with_adjacents"]

@@ -1,56 +1,64 @@
-"""The oracle port (oracle/search.py + oracle/sa_oracle.c) against the REAL reference built into
-oracle/_ref (oracle/build_ref.py) on the seeded synthetic corpus -- the same index object both arms of
-bench.py run on.  Skips where oracle/_ref was never built (it needs /root/reference to build)."""
+"""The oracle port (oracle/search.py + oracle/sa_oracle.c) against the REAL reference on the seeded synthetic
+corpus -- the same index object both arms of bench.py run on.  What the reference returned there is stored in
+tests/golden/ref_cpu.json (made by tests/golden/make_golden_ref_cpu.py from the reference built into oracle/_ref):
+docfreq, and dtype, nonzero count and SHA-256 of every vector, so the comparison stays bit for bit."""
+import hashlib
+import json
+import os
+
 import numpy as np
 import pytest
 
-from oracle import ref_runner
+from conftest import GOLDEN
 
-pytestmark = pytest.mark.skipif(not ref_runner.available(), reason="oracle/_ref not built (python oracle/build_ref.py)")
+G = json.load(open(os.path.join(GOLDEN, "ref_cpu.json")))
 
 
 @pytest.fixture(scope="module")
 def corpus():
     from oracle import search as osearch
     from searcharray_b200 import synth
-    spec = synth.SynthSpec(300_000, terms_per_bucket=5, n_phrases=16, n_bigrams=4)
+    s = G["spec"]
+    spec = synth.SynthSpec(s["n_docs"], terms_per_bucket=s["terms_per_bucket"], n_phrases=s["n_phrases"],
+                           n_bigrams=s["n_bigrams"])
     host, _, _ = synth.generate_shard(spec)
     avgdl = synth.global_avg_doc_length(spec)
-    arr = ref_runner.reference_array(host, avg_doc_length=avgdl)
     oidx = osearch.OracleIndex({t: host.term_words(t) for t in range(host.n_terms)}, host.doc_lens,
                                avg_doc_length=avgdl, corpus_size=host.n_docs, cache=True)
-    return spec, host, arr, oidx
+    return spec, host, oidx
 
 
-def same_bits(a, b):
-    a, b = np.asarray(a), np.asarray(b)
-    return a.dtype == b.dtype and a.shape == b.shape and np.array_equal(a.view(np.uint32), b.view(np.uint32))
+def same_bits(got, rec):
+    got = np.ascontiguousarray(got)
+    return (str(got.dtype) == rec["dtype"] and int(np.count_nonzero(got)) == rec["nonzero"]
+            and hashlib.sha256(got.tobytes()).hexdigest() == rec["sha256"])
 
 
 def test_terms_match_the_reference(corpus):
-    spec, host, arr, oidx = corpus
-    sim = ref_runner.bm25(1.2, 0.75)
+    spec, host, oidx = corpus
+    assert [name for name, _, _ in spec.terms] == list(G["terms"])
     for t, (name, _, _) in enumerate(spec.terms):
-        assert int(arr.docfreq(name)) == int(oidx.docfreq(t))
-        assert same_bits(arr.termfreqs(name), oidx.termfreqs(t)), name
-        assert same_bits(arr.score(name, similarity=sim), oidx.score(t, k1=1.2, b=0.75)), name
-    assert same_bits(arr.score("nope"), oidx.score(None))
+        want = G["terms"][name]
+        assert int(oidx.docfreq(t)) == want["df"]
+        assert same_bits(oidx.termfreqs(t), want["tf"]), name
+        assert same_bits(oidx.score(t, k1=G["k1"], b=G["b"]), want["score"]), name
+    assert same_bits(oidx.score(None), G["missing_term_score"])
 
 
 def test_phrases_and_slop_match_the_reference(corpus):
-    spec, host, arr, oidx = corpus
-    sim = ref_runner.bm25(1.2, 0.75)
+    spec, host, oidx = corpus
+    assert [ph["terms"] for ph in spec.phrases] == [r["terms"] for r in G["phrases"]]
     n_match = 0
-    for ph in spec.phrases:
-        ids = [spec.term_index[t] for t in ph["terms"]]
-        want = arr.termfreqs(ph["terms"])
-        assert same_bits(want, oidx.termfreqs(ids)), ph
-        assert same_bits(arr.score(ph["terms"], similarity=sim), oidx.score(ids, k1=1.2, b=0.75)), ph
-        n_match += int(np.count_nonzero(want))
+    for r in G["phrases"]:
+        ids = [spec.term_index[t] for t in r["terms"]]
+        assert same_bits(oidx.termfreqs(ids), r["tf"]), r["terms"]
+        assert same_bits(oidx.score(ids, k1=G["k1"], b=G["b"]), r["score"]), r["terms"]
+        n_match += r["tf"]["nonzero"]
     assert n_match > 0
     from oracle import ops as oops
-    for ph in spec.phrases[::3]:
-        ids = [spec.term_index[t] for t in ph["terms"]]
-        got = oidx.termfreqs(ids, slop=2)
+    assert [r["terms"] for r in G["slop"]] == [ph["terms"] for ph in spec.phrases[::3]]
+    for r in G["slop"]:
+        ids = [spec.term_index[t] for t in r["terms"]]
+        got = oidx.termfreqs(ids, slop=r["slop"])
         if not oops.last_span_undefined:
-            assert same_bits(arr.termfreqs(ph["terms"], slop=2), got), ph
+            assert same_bits(got, r["tf"]), r["terms"]

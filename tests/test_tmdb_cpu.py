@@ -1,8 +1,7 @@
 """BASELINE configs[0]: the TMDB fixture (27,846 real documents) -- the host indexer and the CPU
 oracle against what the REAL reference produced on it (tests/golden/tmdb.json: digests, counts and
-top-10 lists; made by tests/golden/make_golden_tmdb.py).  The corpus stays in the reference tree, so
-these tests run where /root/reference exists (the build container) and skip elsewhere."""
-import gzip
+top-10 lists; made by tests/golden/make_golden_tmdb.py).  The documents are read back, as token
+sequences, from the fixture's stored index (tests/golden/tmdb_index.npz) and indexed again."""
 import hashlib
 import json
 import os
@@ -10,10 +9,8 @@ import os
 import numpy as np
 import pytest
 
+from _tmdb_index import documents, load_fields
 from conftest import GOLDEN
-
-FIXTURE = "/root/reference/fixtures/tmdb.json.gz"
-pytestmark = pytest.mark.skipif(not os.path.exists(FIXTURE), reason="TMDB fixture lives in the reference tree")
 
 G = json.load(open(os.path.join(GOLDEN, "tmdb.json")))
 
@@ -26,13 +23,9 @@ def sha(a):
 def fields():
     from oracle import search as osearch, solr as osolr
     from searcharray_b200.indexing import build_index
-    with gzip.open(FIXTURE) as f:
-        raw = json.load(f)
-    titles = [(raw[k].get("title", "") or "") for k in raw.keys()]
-    overviews = [(raw[k].get("overview", "") or "") for k in raw.keys()]
     out = {}
-    for name, docs in (("title_tokens", titles), ("overview_tokens", overviews)):
-        host = build_index(docs, str.split)
+    for name, stored in load_fields().items():
+        host = build_index(documents(stored), str.split)
         idx = osearch.OracleIndex({t: host.term_words(t) for t in range(host.n_terms)}, host.doc_lens,
                                   avg_doc_length=host.avg_doc_length)
         out[name] = (host, osolr.OracleField(idx, host.term_dict.term_to_ids))

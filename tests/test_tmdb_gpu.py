@@ -11,6 +11,7 @@ import numpy as np
 import pandas as pd
 import pytest
 
+from _tmdb_index import load_fields
 from conftest import GOLDEN
 
 pytestmark = pytest.mark.gpu
@@ -22,34 +23,11 @@ def sha(a):
     return hashlib.sha256(np.ascontiguousarray(a).tobytes()).hexdigest()
 
 
-def load_field(z, name):
-    from searcharray_b200.indexing import HostIndex, TermDict
-    lengths, offsets = z[name + ".lengths"], z[name + ".offsets"]
-    words = z[name + ".delta"].copy()
-    # undo the per-term delta coding: cumulative sum inside each term's slice
-    starts = offsets[lengths > 0].astype(np.int64)
-    csum = np.cumsum(words, dtype=np.uint64)
-    base = np.zeros(len(words), dtype=np.uint64)
-    order = np.argsort(starts)
-    s_sorted = starts[order]
-    before = np.where(s_sorted > 0, csum[np.maximum(s_sorted, 1) - 1], np.uint64(0))
-    seg_len = np.diff(np.concatenate((s_sorted, [len(words)])))
-    base = np.repeat(before, seg_len)
-    words = csum - base
-    td = TermDict()
-    for t in bytes(z[name + ".terms"]).decode("utf-8").split("\n"):
-        td.add_term(t)
-    return HostIndex(words, offsets, lengths, z[name + ".doc_lens"], td,
-                     avg_doc_length=z[name + ".avg_doc_length"][()])
-
-
 @pytest.fixture(scope="module")
 def frame():
     from searcharray_b200 import SearchArray
-    z = np.load(os.path.join(GOLDEN, "tmdb_index.npz"))
     cols = {}
-    for name in ("title_tokens", "overview_tokens"):
-        host = load_field(z, name)
+    for name, host in load_fields().items():
         want = G["fields"][name]["index"]
         assert (host.n_terms, len(host.words), host.n_docs) == (want["n_terms"], want["n_words"], G["n_docs"])
         cols[name] = SearchArray.from_host_index(host)
