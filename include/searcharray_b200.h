@@ -133,6 +133,11 @@ int sa_batch_upload(sa_index *index, const uint32_t *terms, const uint32_t *term
                     float avg_doc_len, float k1, float b, uint32_t k);
 int sa_batch_execute(sa_index *index);
 int sa_batch_download(sa_index *index, uint32_t *out_docs, float *out_scores, uint32_t *n_overflow);
+/* Diagnostic export: copies dense score row `row` (n_docs floats) of the last chunk that
+ * sa_batch_execute ran into out_host.  A chunk's rows are its single-term queries in query order,
+ * then its phrase queries.  Valid until the next upload or execute, or a download that re-runs a
+ * query exactly (the re-run reuses the rows). */
+int sa_batch_row(sa_index *index, uint32_t row, float *out_host);
 /* CUDA-event timer on the library's own stream (the stream the kernels are launched on). */
 int sa_timer_start(sa_index *index);
 int sa_timer_stop(sa_index *index, double *ms_out);

@@ -51,6 +51,7 @@ SIGNATURES = {
     "sa_batch_upload": (c_int, [P_void, P_u32, P_u32, P_f32, c_u32, c_u32, c_f32, c_f32, c_f32, c_u32]),
     "sa_batch_execute": (c_int, [P_void]),
     "sa_batch_download": (c_int, [P_void, P_u32, P_f32, P_u32]),
+    "sa_batch_row": (c_int, [P_void, c_u32, P_f32]),
     "sa_timer_start": (c_int, [P_void]),
     "sa_timer_stop": (c_int, [P_void, ctypes.POINTER(ctypes.c_double)]),
     "sa_stats_reset": (c_int, [P_void]),

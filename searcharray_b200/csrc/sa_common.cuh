@@ -145,6 +145,10 @@ struct sa_index {
 
     cudaStream_t stream = nullptr;
     cudaEvent_t ev0 = nullptr, ev1 = nullptr;   // sa_timer_start / sa_timer_stop
+    // a batch's top-k selects run here, each overlapping the next chunk's scan (sa_batch_execute_locked); every
+    // batch joins back into `stream` before its last kernel
+    cudaStream_t select_stream = nullptr;
+    cudaEvent_t ev_scan = nullptr, ev_select[2] = {nullptr, nullptr};
     bool profiling = false;
     std::vector<struct TimedLaunch> *pending_timers = nullptr;
     std::vector<cudaEvent_t> *free_events = nullptr;
@@ -182,8 +186,9 @@ struct KernelTimer {
     sa_index *ix;
     int kind;
     bool on;
+    cudaStream_t stream;             // the launch's stream (ix->stream unless given)
     cudaEvent_t e0 = nullptr, e1 = nullptr;
-    KernelTimer(sa_index *ix_, int kind_);
+    KernelTimer(sa_index *ix_, int kind_, cudaStream_t stream_ = nullptr);
     void stop();
 };
 int sa_resolve_timers(sa_index *ix);

@@ -532,6 +532,9 @@ extern "C" int sa_index_destroy(sa_index *ix) {
     if (ix->h_pinned) cudaFreeHost(ix->h_pinned);
     if (ix->ev0) cudaEventDestroy(ix->ev0);
     if (ix->ev1) cudaEventDestroy(ix->ev1);
+    if (ix->ev_scan) cudaEventDestroy(ix->ev_scan);
+    for (cudaEvent_t e : ix->ev_select) if (e) cudaEventDestroy(e);
+    if (ix->select_stream) cudaStreamDestroy(ix->select_stream);
     if (ix->stream) cudaStreamDestroy(ix->stream);
     delete ix;
     return SA_OK;
@@ -705,6 +708,7 @@ struct BatchState {
     u32 nq = 0, k = 0, slots = 0, chunk = 0, slop = 0;
     float avg_doc_len = 0, k1 = 0, b = 0;
     bool ready = false;
+    bool executed = false;                    // the dense rows hold the last chunk (sa_batch_row)
     std::vector<TermQuery> tqs;               // all term queries, chunk by chunk
     std::vector<PhraseQuery> pqs;             // all phrase queries, chunk by chunk
     std::vector<u32> row_query;               // row -> original query index
@@ -740,13 +744,18 @@ TermQuery sa_make_term_query(const sa_index *ix, u32 term_id, float idf) { retur
 static u32 n_tiles_of(const sa_index *ix) { return (u32)((ix->n_docs + SA_TILE_DOCS - 1) / SA_TILE_DOCS); }
 
 static size_t cand_bytes(const sa_index *ix, u32 Q, u32 slots) {
-    return (size_t)Q * n_tiles_of(ix) * ((size_t)slots * sizeof(u64) + 2 * sizeof(u32)) + 64;
+    return ((size_t)Q * n_tiles_of(ix) * ((size_t)slots * sizeof(u64) + 2 * sizeof(u32)) + 255) / 256 * 256;
 }
 
-static TopkCtx make_topk_ctx(sa_index *ix, u32 Q, u32 slots, u32 k, u32 *d_overflow) {
+// A batch alternates between two candidate areas, chunk by chunk: chunk c's select reads area c % 2 while the scan of
+// chunk c + 1 fills the other one.
+static size_t batch_cand_bytes(const sa_index *ix, const BatchState &B) { return 2 * cand_bytes(ix, B.chunk, B.slots); }
+
+// `area`: the candidate area (0 or 1, each cand_bytes(ix, Q, slots) long)
+static TopkCtx make_topk_ctx(sa_index *ix, u32 Q, u32 slots, u32 k, u32 *d_overflow, u32 area = 0) {
     const u32 T = n_tiles_of(ix);
     TopkCtx t;
-    t.tile_cand = ix->cand.as<u64>();
+    t.tile_cand = (u64 *)((char *)ix->cand.p + area * cand_bytes(ix, Q, slots));
     t.tile_cnt = (u32 *)(t.tile_cand + (u64)Q * T * slots);
     t.tile_max = t.tile_cnt + (u64)Q * T;
     t.overflow = d_overflow;
@@ -782,8 +791,16 @@ int sa_batch_upload_locked(sa_index *ix, const uint32_t *terms, const uint32_t *
     SA_CHECK(k >= 1 && k <= SA_TOPK_MAX, "k must be in [1, %d]", SA_TOPK_MAX);
     SA_CUDA(cudaSetDevice(ix->device));
     if (!ix->batch) ix->batch = new BatchState();
+    if (!ix->select_stream) {
+        int least = 0, greatest = 0;        // the selects' few CTAs go ahead of the waiting CTAs of the next scan
+        SA_CUDA(cudaDeviceGetStreamPriorityRange(&least, &greatest));
+        SA_CUDA(cudaStreamCreateWithPriority(&ix->select_stream, cudaStreamNonBlocking, greatest));
+        SA_CUDA(cudaEventCreateWithFlags(&ix->ev_scan, cudaEventDisableTiming));
+        for (cudaEvent_t &e : ix->ev_select) SA_CUDA(cudaEventCreateWithFlags(&e, cudaEventDisableTiming));
+    }
     BatchState &B = *ix->batch;
     B.ready = false;
+    B.executed = false;
     B.nq = n_queries;
     B.k = k;
     B.slots = sa_topk_slots(k);
@@ -798,8 +815,9 @@ int sa_batch_upload_locked(sa_index *ix, const uint32_t *terms, const uint32_t *
     if ((rc = ix->topk_out.reserve(std::max<size_t>(((size_t)n_queries * k + SA_BATCH_TAIL) * sizeof(u64), 256)))) return rc;
     if (n_queries == 0) { B.ready = true; return SA_OK; }
     const u64 stride = padded_docs(std::max<u64>(ix->n_docs, 1));
-    // chunk so the dense score vectors of one chunk stay within ~4 GB of HBM
-    u32 chunk = (u32)std::max<u64>(1, std::min<u64>(n_queries, (4ull << 30) / (stride * sizeof(float))));
+    // chunk so the dense score vectors of one chunk stay within ~16 GB of HBM: at 10M docs 1,024 queries run as 3 scans
+    // of up to 429 queries instead of 10 of 107 (fewer launch tails; 2 % on the bench's mix, profiles/README.md)
+    u32 chunk = (u32)std::max<u64>(1, std::min<u64>(n_queries, (16ull << 30) / (stride * sizeof(float))));
     B.chunk = std::min<u32>(chunk, 65535);
     u64 max_arena = 64;
     size_t max_span_scratch = 0;
@@ -894,7 +912,7 @@ int sa_batch_upload_locked(sa_index *ix, const uint32_t *terms, const uint32_t *
     SA_CHECK(B.chunks.empty() || B.chunks[0].params.sparse_ok || (B.pqs.empty() && n_span == 0),
              "phrase queries in a batch need ordinary BM25 parameters (k1 > 0, 0 <= b < 1, finite idf)");
     if ((rc = ix->dense.reserve((size_t)B.chunk * stride * sizeof(float)))) return rc;
-    if ((rc = ix->cand.reserve(cand_bytes(ix, B.chunk, B.slots)))) return rc;
+    if ((rc = ix->cand.reserve(batch_cand_bytes(ix, B)))) return rc;
     if ((rc = B.d_tq.reserve(std::max<size_t>(B.tqs.size() * sizeof(TermQuery), 64)))) return rc;
     if ((rc = B.d_pq.reserve(std::max<size_t>(B.pqs.size() * sizeof(PhraseQuery), 64)))) return rc;
     if ((rc = B.d_row_query.reserve((size_t)n_queries * sizeof(u32)))) return rc;
@@ -992,9 +1010,13 @@ int sa_batch_execute_locked(sa_index *ix) {
         SA_CUDA(cudaMemsetAsync(B.d_pstats.p, 0, B.pqs.size() * sizeof(PhraseStats), ix->stream));
     int rc;
     size_t chunk_i = 0;
-    for (const BatchChunk &C : B.chunks) {
+    for (size_t c = 0; c < B.chunks.size(); c++) {
+        const BatchChunk &C = B.chunks[c];
         const u32 Q = C.n_term + C.n_phrase;
-        TopkCtx t = make_topk_ctx(ix, Q, B.slots, B.k, d_ovf + C.row0);
+        const u32 area = (u32)(c & 1);
+        // chunk c's scan rewrites the candidate area that chunk c - 2's select reads
+        if (c >= 2) SA_CUDA(cudaStreamWaitEvent(ix->stream, ix->ev_select[area], 0));
+        TopkCtx t = make_topk_ctx(ix, B.chunk, B.slots, B.k, d_ovf + C.row0, area);
         if (C.n_term) {
             TermBatchArgs a = make_term_args(ix, B.d_tq.as<TermQuery>() + C.term0, C.params, t);
             if ((rc = launch_term_batch(ix, a, C.n_term))) return rc;
@@ -1025,8 +1047,16 @@ int sa_batch_execute_locked(sa_index *ix) {
                                         C.n_phrase, rows, stride, C.phrase_chunks, (u64 *)ix->phrase_scratch.p + 8,
                                         d_used, C.arena_words, 1, C.params, &t, C.n_term, &sp))) return rc;
         }
-        if ((rc = launch_topk_select(ix, t, Q, ix->doc_base, d_keys, B.d_row_query.as<u32>() + C.row0))) return rc;
+        // the select runs on the side stream, overlapping the next chunk's scan
+        SA_CUDA(cudaEventRecord(ix->ev_scan, ix->stream));
+        SA_CUDA(cudaStreamWaitEvent(ix->select_stream, ix->ev_scan, 0));
+        if ((rc = launch_topk_select(ix, t, Q, ix->doc_base, d_keys, B.d_row_query.as<u32>() + C.row0, ix->select_stream)))
+            return rc;
+        SA_CUDA(cudaEventRecord(ix->ev_select[area], ix->select_stream));
     }
+    B.executed = true;
+    // join: the summary and everything after it on ix->stream (downloads, timers, the all-gather) follow the selects
+    SA_CUDA(cudaStreamWaitEvent(ix->stream, ix->ev_select[(B.chunks.size() - 1) & 1], 0));
     const u32 n_phr = B.slop > 0 ? 0u : (u32)B.pqs.size();
     batch_summary_kernel<<<1, 256, 0, ix->stream>>>(d_ovf, B.nq, B.d_pq.as<PhraseQuery>(), B.d_pstats.as<PhraseStats>(),
                                                    B.d_missing.as<u32>(), n_phr, d_keys + (size_t)B.nq * B.k);
@@ -1105,10 +1135,11 @@ int sa_batch_fix_overflow_locked(sa_index *ix, u32 *n_redone) {
         }
     }
     if (redo.empty()) return SA_OK;
+    B.executed = false;                          // the re-runs reuse the dense rows
     for (const Redo &r : redo)
         if ((rc = redo_query(ix, B, r.phrase, r.idx, r.q, r.sq))) return rc;
     // the repair buffers are larger than the batch's: restore the normal ones and descriptors
-    if ((rc = ix->cand.reserve(cand_bytes(ix, B.chunk, B.slots)))) return rc;
+    if ((rc = ix->cand.reserve(batch_cand_bytes(ix, B)))) return rc;
     SA_CUDA(cudaMemcpyAsync(B.d_row_query.p, B.row_query.data(), (size_t)B.nq * sizeof(u32), cudaMemcpyHostToDevice, ix->stream));
     if (!B.pqs.empty())
         SA_CUDA(cudaMemcpyAsync(B.d_pq.p, B.pqs.data(), B.pqs.size() * sizeof(PhraseQuery), cudaMemcpyHostToDevice, ix->stream));
@@ -1179,6 +1210,19 @@ extern "C" int sa_batch_download(sa_index *ix, uint32_t *out_docs, float *out_sc
     return sa_batch_download_locked(ix, out_docs, out_scores, n_overflow);
 }
 
+extern "C" int sa_batch_row(sa_index *ix, uint32_t row, float *out_host) {
+    SA_CHECK(ix && out_host, "NULL argument");
+    std::lock_guard<std::mutex> g(ix->mu);
+    SA_CHECK(ix->batch && ix->batch->executed, "no executed batch holds its dense rows");
+    const BatchChunk &C = ix->batch->chunks.back();
+    SA_CHECK(row < C.n_term + C.n_phrase, "row %u out of range (the last chunk has %u)", row, C.n_term + C.n_phrase);
+    SA_CUDA(cudaSetDevice(ix->device));
+    SA_CUDA(cudaMemcpyAsync(out_host, ix->dense.as<float>() + (u64)row * padded_docs(ix->n_docs), ix->n_docs * sizeof(float),
+                            cudaMemcpyDeviceToHost, ix->stream));
+    SA_CUDA(cudaStreamSynchronize(ix->stream));
+    return SA_OK;
+}
+
 extern "C" int sa_score_batch_topk(sa_index *ix, const uint32_t *terms, const uint32_t *term_starts,
                                    const float *idf, uint32_t n_queries, uint32_t slop,
                                    float avg_doc_len, float k1, float b, uint32_t k,
@@ -1192,7 +1236,8 @@ extern "C" int sa_score_batch_topk(sa_index *ix, const uint32_t *terms, const ui
 }
 
 // ------------------------------------------------------------------- timers
-KernelTimer::KernelTimer(sa_index *ix_, int kind_) : ix(ix_), kind(kind_), on(ix_->profiling) {
+KernelTimer::KernelTimer(sa_index *ix_, int kind_, cudaStream_t stream_)
+    : ix(ix_), kind(kind_), on(ix_->profiling), stream(stream_ ? stream_ : ix_->stream) {
     if (!on) return;
     if (!ix->pending_timers) ix->pending_timers = new std::vector<TimedLaunch>();
     if (!ix->free_events) ix->free_events = new std::vector<cudaEvent_t>();
@@ -1204,12 +1249,12 @@ KernelTimer::KernelTimer(sa_index *ix_, int kind_) : ix(ix_), kind(kind_), on(ix
     };
     e0 = get();
     e1 = get();
-    cudaEventRecord(e0, ix->stream);
+    cudaEventRecord(e0, stream);
 }
 
 void KernelTimer::stop() {
     if (!on) return;
-    cudaEventRecord(e1, ix->stream);
+    cudaEventRecord(e1, stream);
     ix->pending_timers->push_back(TimedLaunch{e0, e1, kind});
     on = false;
 }

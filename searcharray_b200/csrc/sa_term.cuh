@@ -6,7 +6,7 @@
 #define SA_TERM_UNROLL 4           // 30-word windows loaded per warp before processing
 #define SA_TERM_THREADS 256
 #define SA_STAGED_NORM_MIN_WORDS 1024   // tiles with at least this many posting words stage the tile's norms (sa_term.cu)
-#define SA_STAGED_NORM_MIN_RECS 48      // ... or this many (doc, tf) records on the tf-table path
+#define SA_STAGED_NORM_MIN_RECS 96      // ... or this many (doc, tf) records on the tf-table path
 #define SA_TERM_PREFETCH_TILES 8         // L2 prefetch distance of the tf-table path, in tiles (sa_term.cu)
 #define SA_TERM_QUAD_MIN_RECS 512       // four records per thread from this many records per tile on (and >= 16 * k, sa_term.cu)
 #define SA_TOPK_MAX 32             // warp-level threshold estimation handles k <= 32
@@ -51,7 +51,7 @@ struct TermBatchArgs {
 int launch_term_batch(sa_index *ix, const TermBatchArgs &a, u32 n_queries);
 int sa_ensure_norm(sa_index *ix, float k1, float b, float avg_doc_len);
 int launch_topk_select(sa_index *ix, const TopkCtx &t, u32 n_queries, u64 doc_base, u64 *d_out_keys,
-                       const u32 *d_out_index);
+                       const u32 *d_out_index, cudaStream_t stream = nullptr);   // nullptr: ix->stream
 u32 sa_topk_slots(u32 k);
 Bm25Params sa_make_bm25(const sa_index *ix, float idf, float avg_doc_len, float k1, float b);
 TermQuery sa_make_term_query(const sa_index *ix, u32 term_id, float idf);

@@ -196,10 +196,11 @@ topk_merge_kernel(const u64 *__restrict__ in, u64 rank_stride, u32 world, u32 n_
 }
 
 int launch_topk_select(sa_index *ix, const TopkCtx &t, u32 n_queries, u64 doc_base, u64 *d_out_keys,
-                       const u32 *d_out_index) {
+                       const u32 *d_out_index, cudaStream_t stream) {
     if (n_queries == 0) return SA_OK;
-    KernelTimer tm(ix, 1);
-    topk_select_kernel<<<n_queries, SEL_THREADS, 0, ix->stream>>>(t, doc_base, d_out_keys, d_out_index);
+    if (!stream) stream = ix->stream;
+    KernelTimer tm(ix, 1, stream);
+    topk_select_kernel<<<n_queries, SEL_THREADS, 0, stream>>>(t, doc_base, d_out_keys, d_out_index);
     SA_CUDA(cudaGetLastError());
     tm.stop();
     ix->stats.topk_kernel_launches++;
